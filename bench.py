@@ -97,7 +97,13 @@ def parse():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: --points per GPU; strong: --points in total, split over the GPUs")
     ap.add_argument("--cpu-threads", type=int, default=0, help="host threads of the CPU arm (0: all usable)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what they computed (the refined parameters and the cost of every LM "
+                         "iteration; rank 0's shard of the points) as DIR/<name>.npy, to compare two builds output for output. "
+                         "The solve sums with fp64 atomics, so two runs agree to a tolerance, not bit for bit")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path: use it with --impl b200")
     if args.workload == "configs4":
         # 5k cams / 2M pts / 20M obs over 8 GPUs = 250k pts / 2.5M obs per GPU; 8x8 patches (41 GB per GPU instead of 164 GB)
         d = ap.parse_args([])
@@ -211,6 +217,22 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm), "samples_in_timed_region": inside,
                 "window": "start of warm-up .. end of timed region (+50 ms)", "period_ms": self.period_ms,
                 "source": "NVML" if getattr(self, "nvml", None) else "nvidia-smi"}
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(dirname, arrays):
+    """Each array as DIR/<name>.npy in float64.  An array larger than its share of DUMP_BYTES is replaced by the same
+    seeded sample of its rows on every run, so that two runs with the same arguments write comparable files."""
+    os.makedirs(dirname, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 1024            # room for the .npy header
+    for name, a in arrays.items():
+        a = np.asarray(a, np.float64)
+        if a.nbytes > share:
+            rows = np.random.default_rng(0).choice(len(a), share // (a.nbytes // len(a)), replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def geometry(args, rank):
@@ -535,6 +557,10 @@ def main():
             stage_ms[nm] = {"ms_per_step": tms / max(1, args.steps), "launch_groups": tn}
     k1_ms, k1_n = h.kernel_timing(enable=0, which=1)
     its = s["iterations"][1:] if args.steps > 0 else []
+    if args.dump_outputs and rank == 0:
+        h.read_params()                                    # the parameters a solve of K iterations hands back
+        dump_outputs(args.dump_outputs, {"cam_params": prob.cam_params, "qvec": prob.qvec, "tvec": prob.tvec, "xyz": prob.xyz,
+                                         "iteration_cost": [i["cost"] for i in s["iterations"]]})
     steps_done = len(its)
     total_obs = n_obs * world
     value = total_obs * steps_done / (ms / 1e3) if ms > 0 else 0.0

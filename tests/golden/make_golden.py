@@ -1,9 +1,9 @@
 """Generates tests/golden/*.npz from the reference's OWN code (oracle/_ref/libpxref.so =
-pixsfm/base/src/cubic_hermite_spline_simd.h + pixsfm/base/src/graph.cc compiled verbatim from
-/root/reference by oracle/Makefile).  Run in the build container only:
-    python tests/golden/make_golden.py
-The fixtures pin the oracle's restatement (tests/test_oracle_golden.py) on boxes where
-/root/reference does not exist."""
+pixsfm/base/src/cubic_hermite_spline_simd.h + pixsfm/base/src/graph.cc compiled verbatim by
+oracle/Makefile from a reference checkout, REF=<path>).  Needs that library:
+    python tests/golden/make_golden.py [spline graph spline_live]
+(no argument: all fixtures).  The fixtures pin the oracle's restatement (tests/test_oracle_golden.py)
+wherever the reference checkout is absent."""
 import ctypes as C
 import os
 import sys
@@ -64,7 +64,20 @@ def graph_fixture():
     np.savez_compressed(os.path.join(HERE, "graph_ref.npz"), **out)
 
 
+def spline_live_fixture():
+    """the input of test_live_reference_library_if_present and the reference's answer on it"""
+    rng = np.random.default_rng(99)
+    P = rng.uniform(-1, 1, (4, 4, 128)).astype(np.float16)
+    x = rng.uniform(0, 1, 4)
+    F = np.zeros((4, 128)); D = np.zeros((4, 128))
+    for i in range(4):
+        rc = ref.ref_spline_f16(128, p(P[i, 0]), p(P[i, 1]), p(P[i, 2]), p(P[i, 3]), C.c_double(x[i]), p(F[i]), p(D[i]))
+        assert rc == 0
+    np.savez_compressed(os.path.join(HERE, "spline_live_ref.npz"), P=P, x=x, f=F, d=D)
+
+
 if __name__ == "__main__":
-    spline_fixture()
-    graph_fixture()
+    fixtures = {"spline": spline_fixture, "graph": graph_fixture, "spline_live": spline_live_fixture}
+    for name in sys.argv[1:] or fixtures:
+        fixtures[name]()
     print("wrote", os.listdir(HERE))

@@ -1,7 +1,7 @@
-"""util/h5lite.py — the classic-layout HDF5 subset in pure Python.  Read side against REAL HDF5 files: the reference tree
-ships ten h5py-written calibration files (datasets/sacre_coeur/ground_truth/calibration_*.h5; one of them is kept as
-tests/golden/calibration_sample.h5 so the check also runs where /root/reference is absent).  Their content is
-self-checking: K is an intrinsics matrix, R a rotation, q the same rotation as a unit quaternion.  Write side: round trips
+"""util/h5lite.py — the classic-layout HDF5 subset in pure Python.  Read side against REAL HDF5 files: the ten
+h5py-written calibration files the reference ships with its sacre_coeur dataset (datasets/sacre_coeur/ground_truth/),
+kept under tests/golden/calibration/.  Their content is self-checking: K is an intrinsics matrix, R a rotation, q the
+same rotation as a unit quaternion.  Write side: round trips
 (nested groups, many links, chunked patches, attributes), and the hloc / feature-cache helpers on top of it."""
 import glob
 import os
@@ -32,8 +32,9 @@ def _check_calibration(path):
 
 
 def test_reads_real_hdf5_files():
-    _check_calibration(os.path.join(HERE, "golden", "calibration_sample.h5"))
-    for path in sorted(glob.glob("/root/reference/datasets/sacre_coeur/ground_truth/calibration_*.h5")):
+    paths = sorted(glob.glob(os.path.join(HERE, "golden", "calibration", "calibration_*.h5")))
+    assert len(paths) == 10
+    for path in paths:
         _check_calibration(path)
 
 

@@ -1,6 +1,7 @@
 """use_nonmonotonic_steps (ceres::Solver::Options; the reference's configs/default.yaml switches it on for KA, BA and
-QKA): the oracle's restatement of ceres' TrustRegionStepEvaluator, the reference YAML files taken as far as the solver
-options of every optimizer, and (GPU) the device LM drivers against the oracle with the option on."""
+QKA): the oracle's restatement of ceres' TrustRegionStepEvaluator, the reference YAML files (configs/default.yaml and
+low_memory.yaml, kept under tests/golden/configs/) taken as far as the solver options of every optimizer, and (GPU) the
+device LM drivers against the oracle with the option on."""
 import os
 
 import numpy as np
@@ -10,7 +11,7 @@ import oracle_lib as O
 from pixsfm._pixsfm import _capi
 from pixsfm.util import synthetic
 
-REF_CONFIGS = "/root/reference/pixsfm/configs"
+REF_CONFIGS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "configs")
 
 
 def _hard_ba_problem(seed=4):
@@ -42,7 +43,6 @@ def test_monotonic_evaluator_is_the_old_rule_and_nonmonotonic_returns_the_best_i
     assert abs(O.ba_evaluate(p_m, ic, so)["cost"] - s_m["final_cost"]) <= 1e-12 * s_m["final_cost"]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CONFIGS), reason="reference checkout not present")
 @pytest.mark.parametrize("name", ["default.yaml", "low_memory.yaml"])
 def test_reference_yaml_reaches_the_solver_options(name):
     """ADVICE r1: PixSfM(<reference yaml>) must not only construct but also yield solver options for every optimizer"""
