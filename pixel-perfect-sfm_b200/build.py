@@ -6,7 +6,7 @@ from concurrent.futures import ThreadPoolExecutor
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
-SOURCES = ["pxr_api.cu", "pxr_upload.cu", "pxr_ba.cu", "pxr_ba_block.cu", "pxr_inner.cu", "pxr_refs.cu", "pxr_ka.cu", "pxr_synth.cu", "pxr_extract.cu", "pxr_problem.cu"]
+SOURCES = ["pxr_api.cu", "pxr_upload.cu", "pxr_ba.cu", "pxr_ba_block.cu", "pxr_refs.cu", "pxr_ka.cu", "pxr_synth.cu", "pxr_extract.cu", "pxr_problem.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC", "-ccbin", "/usr/bin/g++", "--expt-relaxed-constexpr",

@@ -92,6 +92,47 @@ int launch_fm_eval(pxr_ctx* ctx, int dtype, int C, int mode, bool float_simd, co
   return fail(PXR_ERR_UNSUPPORTED, "Unsupported dimensions (CHANNELS=%d, dtype=%d, N_NODES=1).", C, dtype);
 }
 
+// -------------------------------------------------------------------------------- inner iterations dispatch
+template <typename T, int C, bool FS>
+static int launch_inner_k(pxr_ctx* ctx, const InnerArgs& a) {
+  typedef InnerCfg<T, C> Cfg;
+  auto kern = inner_fused_kernel<T, C, FS>;
+  static bool attr_set = false;
+  if (!attr_set) {
+    PXR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmem));
+    attr_set = true;
+  }
+  // two CTAs per SM (the L2 budget of pxr_inner.cuh); fewer when there are fewer points
+  const int64_t grid = std::max<int64_t>(1, std::min<int64_t>((int64_t)ctx->sm_count * 2, cdiv(a.n_points, kInnerSlots)));
+  PXR_LAUNCH(ctx, kern, (unsigned)grid, Cfg::kWarps * 32, Cfg::kSmem, a);
+  PXR_CUDA(cudaGetLastError());
+  return PXR_OK;
+}
+
+// the (dtype, C) pairs of launch_fm_eval
+int launch_inner_fused(pxr_ctx* ctx, int dtype, int C, bool float_simd, const InnerArgs& a) {
+#define PXR_SMALL(T) \
+  { if (C == 3) return launch_inner_k<T, 3, false>(ctx, a); if (C == 4) return launch_inner_k<T, 4, false>(ctx, a); \
+    if (C == 1) return launch_inner_k<T, 1, false>(ctx, a); }
+  if (C < 8) {
+    if (dtype == PXR_F16) PXR_SMALL(__half) else if (dtype == PXR_F32) PXR_SMALL(float) else if (dtype == PXR_F64) PXR_SMALL(double)
+    return fail(PXR_ERR_UNSUPPORTED, "Unsupported dimensions (CHANNELS=%d, dtype=%d, N_NODES=1).", C, dtype);
+  }
+#undef PXR_SMALL
+#define PXR_CASE(T, CC) \
+  if (C == CC) return float_simd ? launch_inner_k<T, CC, true>(ctx, a) : launch_inner_k<T, CC, false>(ctx, a);
+  if (dtype == PXR_F16) {
+    PXR_CASE(__half, 128) PXR_CASE(__half, 64) PXR_CASE(__half, 32) PXR_CASE(__half, 16) PXR_CASE(__half, 8)
+    PXR_CASE(__half, 256)
+  } else if (dtype == PXR_F32) {
+    PXR_CASE(float, 128) PXR_CASE(float, 64) PXR_CASE(float, 16)
+  } else if (dtype == PXR_F64) {
+    PXR_CASE(double, 128) PXR_CASE(double, 16)
+  }
+#undef PXR_CASE
+  return fail(PXR_ERR_UNSUPPORTED, "Unsupported dimensions (CHANNELS=%d, dtype=%d, N_NODES=1).", C, dtype);
+}
+
 // -------------------------------------------------------------------------------- problem upload
 static int check_desc(const pxr_ba_desc* d) {
   if (!d) return fail(PXR_ERR_INVALID_ARGUMENT, "desc is NULL");
@@ -286,7 +327,6 @@ int BA::create(pxr_ctx* c, const pxr_ba_desc* d, const pxr_interp_config* ic, co
   PXR_TRY(gc.alloc(nc));
   PXR_TRY(Hpp.alloc((size_t)n_points * 9)); PXR_TRY(gp.alloc((size_t)n_points * 3));
   h_obs_img.assign(d->obs_img, d->obs_img + n_obs);
-  use_monolithic_inner = std::getenv("PXR_INNER_MONOLITHIC") != nullptr;
   if (for_solve) PXR_TRY(build_schur_pairs());
   if (block_mode) PXR_TRY(block_setup());
   if (for_solve && n_obs > 0 && n_obs < ((int64_t)1 << 31)) {
@@ -479,7 +519,6 @@ int BA::resident_setup(const pxr_ba_desc* d, size_t esz) {
   const int W = res_window;
   if (W < 4 || C < 8 || ph > 255 || pw > 255 || ph < W + 2 || pw < W + 2) return PXR_OK;       // nothing to gain / not representable
   if ((size_t)ph * pw * C * esz > staged_chunk_bytes()) return PXR_OK;      // a whole (shared) patch must fit a staging buffer
-  if (getenv("PXR_INNER_MONOLITHIC")) return PXR_OK;     // that kernel reads taps without the residency guard
   // the blocks must be HOST memory (a device-resident block needs no upload at all)
   auto is_device = [](const void* ptr) -> bool {
     cudaPointerAttributes pa;
@@ -570,8 +609,8 @@ int BA::resident_fix(int64_t* n_fixed) {
   PXR_CUDA(cudaMemsetAsync(res_viol_count.p, 0, sizeof(unsigned long long), s));
   PXR_CUDA(cudaStreamSynchronize(s));
   const size_t patch_bytes = (size_t)ph * pw * C * res_esz;
-  // an observation is reported by every pass that evaluates it before its patch is whole (several inner-iteration rounds
-  // run between two looks at the list): fetch each patch once
+  // an observation is reported by every evaluation of it before its patch is whole (the inner iterations evaluate it
+  // many times before the list is looked at): fetch each patch once
   if (res_whole.size() != (size_t)n_patches) res_whole.assign((size_t)n_patches, 0);
   int64_t fetched = 0;
   for (int64_t o : list) {
@@ -635,6 +674,11 @@ int BA::evaluate(int set, bool jac, double* cost_out) {
   PXR_TRY(project(set, jac, nullptr));
   PXR_TRY(fm(jac ? 1 : 0, nullptr, scalars.p + 0));
   if (jac) PXR_TRY(build());
+  return read_cost(cost_out);
+}
+
+// the global cost from this rank's part in scalars[0]
+int BA::read_cost(double* cost_out) {
   if (block_mode) return global_cost_block(cost_out);
   PXR_TRY(allreduce_f64(ctx, scalars.p + 0, 1));
   double c = 0;
@@ -950,117 +994,46 @@ int BA::apply_step(double* step_norm, double* x_norm) {
   return PXR_OK;
 }
 
-// K0 (with Jacobians) + K1 (Jacobian mode) over an explicit list of observations.  With n_dev the number of entries is
-// read on the device (n is then the upper bound the grids are sized for); settle = false leaves the window-residency
-// check to the caller (inner_rounds checks once per batch of rounds).
-int BA::eval_list(int set, const int64_t* list, int64_t n, const unsigned long long* n_dev, bool settle) {
-  if (n <= 0) return PXR_OK;
-  ProjectArgs pa;
-  pa.obs_img = obs_img.p; pa.obs_pt = obs_pt.p; pa.obs_patch = obs_patch.p;
-  pa.img_cam = img_cam.p; pa.cam_model = cam_model.p;
-  pa.cam_params = cam[set].p; pa.qvec = q[set].p; pa.tvec = t[set].p; pa.xyz = X[set].p;
-  pa.corner = corner.p; pa.scale = scale.p; pa.ups = ups;
-  pa.obs_begin = 0; pa.obs_end = n; pa.item_index = list; pa.n_dev = n_dev;
-  pa.uv = uv.p; pa.xy = nullptr; pa.juv = juv.p; pa.juv_stride = juv_stride; pa.juv_k = K;
-  PXR_LAUNCH(ctx, ba_project_kernel<true>, (unsigned)cdiv(n, 128), 128, 0, pa);
-  FmEvalArgs a;
-  a.uv = uv.p; a.item_patch = obs_patch.p; a.item_ref = obs_pt.p;
-  a.patches = d_patches; a.ph = ph; a.pw = pw;
-  a.refs = has_refs ? refs.p : nullptr;
-  a.begin = 0; a.end = n; a.item_index = list; a.end_dev = n_dev;
-  a.out = obs_out.p; a.residuals = nullptr; a.desc = nullptr;
-  a.loss.type = opt.loss_type; a.loss.a = opt.loss_scale;
-  a.l2_normalize = interp.l2_normalize;
-  resident_args(a);
-  int np = 0;
-  PXR_TRY(launch_fm_eval(ctx, dtype, C, 1, interp.use_float_simd != 0, a, &np));
-  if (!settle) return PXR_OK;
-  for (;;) {     // window residency: whoever consumes these results right away needs them settled first
-    int64_t n_fixed = 0;
-    PXR_TRY(resident_fix(&n_fixed));
-    if (n_fixed == 0) break;
-    a.item_index = res_fix_list.p; a.begin = 0; a.end = n_fixed; a.end_dev = nullptr;
-    PXR_TRY(launch_fm_eval(ctx, dtype, C, 1, interp.use_float_simd != 0, a, &np));
-  }
-  return PXR_OK;
-}
-
-// Inner iterations, batched: see pxr_inner.cuh.  Same state machine as ba_inner_kernel.
-// The rounds are enqueued WITHOUT waiting for the host: the list length of a round stays on the device (K0 / K1 read it
-// there, their grids are sized for all observations), its copy travels to a pinned slot behind an event, and the host
-// stops enqueuing once a round two behind has reported an empty list (the two extra rounds find nothing to do).
-constexpr int kInnerRounds = 53;
-int BA::inner_rounds(int set) {
-  cudaStream_t s = ctx->stream;
-  InnerStepArgs a;
-  a.n_points = n_points; a.point_off = point_off.p; a.pt_begin = pt_begin.p;
-  a.obs_out = obs_out.p; a.juv = juv.p; a.juv_stride = juv_stride; a.juv_w = 9 + K;
-  a.xyz = X[set].p; a.st = inner_state.p;
-  a.loss.type = opt.loss_type; a.loss.a = opt.loss_scale;
-  a.list = inner_list.p; a.counters = inner_counters.p;
-  const unsigned pgrid = (unsigned)cdiv(n_points, 128);
-  for (int round = 0; round < kInnerRounds; ++round) {
-    if (round >= 2) {
-      const cudaError_t q = cudaEventQuery(inner_events[round - 2]);
-      if (q == cudaSuccess) { if (inner_cnt_host[2 * (round - 2)] == 0) break; }
-      else if (q != cudaErrorNotReady) PXR_CUDA(q);
-      else if ((void)cudaGetLastError(), round >= 8 && (round & 3) == 0) {        // far ahead of the device: let it catch up rather than pile up empty rounds
-        PXR_CUDA(cudaEventSynchronize(inner_events[round - 2]));
-        if (inner_cnt_host[2 * (round - 2)] == 0) break;
-      }
-    }
-    PXR_CUDA(cudaMemsetAsync(inner_counters.p, 0, 2 * sizeof(unsigned long long), s));
-    PXR_LAUNCH(ctx, inner_list_kernel, pgrid, 128, 0, a, round == 0 ? 1 : 0);
-    PXR_CUDA(cudaMemcpyAsync(inner_cnt_host + 2 * round, inner_counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
-    PXR_CUDA(cudaEventRecord(inner_events[round], s));
-    PXR_TRY(eval_list(set, inner_list.p, n_obs, inner_counters.p, false));
-    PXR_LAUNCH(ctx, inner_step_kernel, pgrid, 128, 0, a, round == 0 ? 0 : 1);
-  }
-  PXR_CUDA(cudaGetLastError());
-  return PXR_OK;
-}
-
-int BA::inner_iterations_batched(int set) {
+// Inner iterations: one launch of inner_fused_kernel (pxr_inner.cuh) solves every variable point with the cameras
+// of parameter set `set` fixed.  It leaves in obs_out[o*8] the squared norm of every observation of those points at
+// the point's final position, so the cost after the inner iterations is fm_cost() over obs_out.
+int BA::inner_iterations(int set) {
   if (n_points == 0 || n_obs == 0) return PXR_OK;
   StageScope stg(this, 9);
   cudaStream_t s = ctx->stream;
-  if (!inner_state.p) {
-    PXR_TRY(inner_state.alloc(n_points));
-    PXR_TRY(inner_list.alloc(n_obs));
-    PXR_TRY(inner_counters.alloc(2));
-    PXR_CUDA(cudaHostAlloc((void**)&inner_cnt_host, (size_t)kInnerRounds * 2 * sizeof(unsigned long long), cudaHostAllocDefault));
-    inner_events.resize(kInnerRounds, nullptr);
-    for (auto& e : inner_events) PXR_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+  if (!inner_rec.p) { PXR_TRY(inner_rec.alloc((size_t)n_obs * kInnerRec)); PXR_TRY(inner_next.alloc(1)); }
+  InnerArgs a;
+  a.n_points = n_points; a.point_off = point_off.p; a.pt_begin = pt_begin.p;
+  a.geo.obs_img = obs_img.p; a.geo.obs_pt = obs_pt.p; a.geo.obs_patch = obs_patch.p;
+  a.geo.img_cam = img_cam.p; a.geo.cam_model = cam_model.p;
+  a.geo.cam_params = cam[set].p; a.geo.qvec = q[set].p; a.geo.tvec = t[set].p; a.geo.xyz = X[set].p;
+  a.geo.corner = corner.p; a.geo.scale = scale.p; a.geo.ups = ups;
+  a.geo.obs_begin = 0; a.geo.obs_end = n_obs; a.geo.item_index = nullptr;
+  a.geo.uv = nullptr; a.geo.xy = nullptr; a.geo.juv = nullptr; a.geo.juv_stride = juv_stride; a.geo.juv_k = K;
+  a.fm.uv = nullptr; a.fm.item_patch = obs_patch.p; a.fm.item_ref = obs_pt.p;
+  a.fm.patches = d_patches; a.fm.ph = ph; a.fm.pw = pw;
+  a.fm.refs = has_refs ? refs.p : nullptr;
+  a.fm.begin = 0; a.fm.end = n_obs; a.fm.item_index = nullptr;
+  a.fm.out = obs_out.p; a.fm.residuals = nullptr; a.fm.desc = nullptr;
+  a.fm.loss.type = opt.loss_type; a.fm.loss.a = opt.loss_scale;
+  a.fm.l2_normalize = interp.l2_normalize;
+  resident_args(a.fm);
+  a.xyz = X[set].p; a.rec = inner_rec.p; a.next_point = inner_next.p;
+  // window residency: an observation may leave its window in any evaluation and nobody looks before the kernel is
+  // over — keep the starting points, and if something was reported fetch those patches and run again from the start
+  if (resident) {
+    if (!inner_snapshot.p) PXR_TRY(inner_snapshot.alloc((size_t)n_points * 3));
+    PXR_CUDA(cudaMemcpyAsync(inner_snapshot.p, X[set].p, (size_t)n_points * 24, cudaMemcpyDeviceToDevice, s));
   }
-  if (!resident) return inner_rounds(set);
-  // window residency: an observation may leave its window in any round and nobody looks before the rounds are over — keep
-  // the starting points, and if something was reported fetch those patches and run the rounds again from the start
-  if (!inner_snapshot.p) PXR_TRY(inner_snapshot.alloc((size_t)n_points * 3));
-  PXR_CUDA(cudaMemcpyAsync(inner_snapshot.p, X[set].p, (size_t)n_points * 24, cudaMemcpyDeviceToDevice, s));
   for (;;) {
-    PXR_TRY(inner_rounds(set));
+    PXR_CUDA(cudaMemsetAsync(inner_next.p, 0, sizeof(unsigned long long), s));
+    PXR_TRY(launch_inner_fused(ctx, dtype, C, interp.use_float_simd != 0, a));
     int64_t n_fixed = 0;
     PXR_TRY(resident_fix(&n_fixed));
     if (n_fixed == 0) break;
     PXR_CUDA(cudaMemcpyAsync(X[set].p, inner_snapshot.p, (size_t)n_points * 24, cudaMemcpyDeviceToDevice, s));
   }
   return PXR_OK;
-}
-
-int BA::inner_iterations(int set) {
-  if (!use_monolithic_inner) return inner_iterations_batched(set);
-  InnerArgs a;
-  a.n_points = n_points; a.point_off = point_off.p; a.pt_begin = pt_begin.p;
-  a.obs_img = obs_img.p; a.obs_patch = obs_patch.p; a.img_cam = img_cam.p; a.cam_model = cam_model.p;
-  a.cam_params = cam[set].p; a.qvec = q[set].p; a.tvec = t[set].p; a.xyz = X[set].p;
-  a.corner = corner.p; a.scale = scale.p; a.ups = ups;
-  a.patches = d_patches; a.ph = ph; a.pw = pw;
-  a.refs = has_refs ? refs.p : nullptr;
-  a.loss.type = opt.loss_type; a.loss.a = opt.loss_scale;
-  a.l2_normalize = interp.l2_normalize;
-  if (n_points == 0) return PXR_OK;
-  StageScope st(this, 9);
-  return launch_inner(ctx, dtype, C, interp.use_float_simd != 0, a);
 }
 
 int BA::step_norm_between_sets(double* out) {
@@ -1339,7 +1312,8 @@ int BA::lm_iterate(int max_iteration) {
       ++lm.n_inner;
       rc = inner_iterations(1 - cur);
       double inner_cost = 0;
-      if (rc == PXR_OK) rc = evaluate(1 - cur, false, &inner_cost);
+      if (rc == PXR_OK) rc = fm_cost(scalars.p + 0);
+      if (rc == PXR_OK) rc = read_cost(&inner_cost);
       if (rc != PXR_OK) { swap_sets(); return rc; }
       if (std::isfinite(inner_cost)) {
         model_cost_change += candidate_cost - inner_cost;

@@ -563,8 +563,7 @@ int BA::lm_iterate_block(int max_iteration) {
       // ceres skips them when the trial cost is not finite — a GLOBAL fact that is only known after the exchange; they are
       // per-point and local, so they run regardless and their result is ignored in that case (the step is rejected)
       rc = inner_iterations(1 - cur);
-      if (rc == PXR_OK) rc = project(1 - cur, false, nullptr);
-      if (rc == PXR_OK) rc = fm(0, nullptr, scalars.p + 0);
+      if (rc == PXR_OK) rc = fm_cost(scalars.p + 0);
       if (rc != PXR_OK) { swap_sets(); return rc; }
       PXR_CUDA(cudaMemsetAsync(scalars.p + 11, 0, 16, s));
       auto run = [&](const double* a, const double* b, int64_t n, double* acc) {

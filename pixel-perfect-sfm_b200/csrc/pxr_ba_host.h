@@ -25,7 +25,7 @@ namespace pxr {
 int fm_supported(int dtype, int C);
 int fm_max_partials(pxr_ctx* ctx);
 int launch_fm_eval(pxr_ctx* ctx, int dtype, int C, int mode, bool float_simd, const FmEvalArgs& a, int* n_partials);
-int launch_inner(pxr_ctx* ctx, int dtype, int C, bool float_simd, const InnerArgs& a);
+int launch_inner_fused(pxr_ctx* ctx, int dtype, int C, bool float_simd, const InnerArgs& a);
 
 // ceres::internal::TrustRegionStepEvaluator (Conn, Gould & Toint, algorithm 10.1.2); max_nonmonotonic == 0 is the
 // monotonic minimizer.  Same arithmetic as oracle/orc_trust_region.h::StepEvaluator.
@@ -179,7 +179,7 @@ struct BA {
   DevBuf<int64_t> io_chunk_begin; int64_t io_n_chunks = 0;
   DevBuf<long long> chol_trace;     // PXR_CHOL_TRACE=<file>: panel-CTA time stamps
   DevBuf<int> chol_sync;            // flags of the persistent tile-DAG Cholesky (pxr_chol.cuh)
-  ~BA() { if (inner_cnt_host) cudaFreeHost(inner_cnt_host); for (auto e : inner_events) cudaEventDestroy(e); if (res_thread.joinable()) res_thread.join(); if (chol_graph_exec) cudaGraphExecDestroy(chol_graph_exec); for (int k = 0; k < kNumStages; ++k) for (auto& pr : timed[k]) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); } }
+  ~BA() { if (res_thread.joinable()) res_thread.join(); if (chol_graph_exec) cudaGraphExecDestroy(chol_graph_exec); for (int k = 0; k < kNumStages; ++k) for (auto& pr : timed[k]) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); } }
   // static co-visibility structure for the Schur complement (see ba_schur_pairs_kernel)
   DevBuf<int32_t> sp_px, sp_py, sp_pp;
   DevBuf<int64_t> sp_chunk_begin;
@@ -221,21 +221,15 @@ struct BA {
   int fm_cost(double* cost_dev);                                                                   // robustified cost from obs_out
   int build();
   int evaluate(int set, bool jac, double* cost_out);
+  int read_cost(double* cost_out);                 // global cost from scalars[0] (all-reduce + read-back)
   int compute_step(double radius, bool* valid, double* model_cost_change);
   int chol_launch();
   int apply_step(double* step_norm, double* x_norm);
   int gradient_max_norm(double* out);
   int inner_iterations(int set);
-  int inner_iterations_batched(int set);
-  int eval_list(int set, const int64_t* list, int64_t n, const unsigned long long* n_dev = nullptr, bool settle = true);
-  int inner_rounds(int set);                       // the <= 52 rounds of inner_iterations_batched, without a host wait per round
-  unsigned long long* inner_cnt_host = nullptr;    // pinned [kInnerRounds][2]: the rounds' list counts, read back asynchronously
-  std::vector<cudaEvent_t> inner_events;
-  DevBuf<double> inner_snapshot;                   // window residency: the points before a batch of rounds (redo after a refetch)
-  DevBuf<InnerState> inner_state;
-  DevBuf<int64_t> inner_list;
-  DevBuf<unsigned long long> inner_counters;
-  bool use_monolithic_inner = false;
+  DevBuf<double> inner_rec;                        // [n_obs][kInnerRec]: the evaluations of a round (pxr_inner.cuh)
+  DevBuf<unsigned long long> inner_next;           // next point a slot of inner_fused_kernel takes
+  DevBuf<double> inner_snapshot;                   // window residency: the points before the inner iterations (redo after a refetch)
   int step_norm_between_sets(double* out);
   int lm_begin();
   bool lm_finalize(int max_iteration);

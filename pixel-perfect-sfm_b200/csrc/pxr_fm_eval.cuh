@@ -27,9 +27,7 @@ struct ProjectArgs {
   const double* cam_params; const double* qvec; const double* tvec; const double* xyz;
   const int32_t* corner; const double* scale; double ups;
   int64_t obs_begin, obs_end;
-  const int64_t* item_index;  // optional: process observations item_index[obs_begin..obs_end) (inner iterations)
-  const unsigned long long* n_dev = nullptr;   // optional: the item count lives on the device (obs_end = obs_begin + *n_dev; the
-                                               // grid is sized for an upper bound) — no host round trip between list and launch
+  const int64_t* item_index;  // optional: process observations item_index[obs_begin..obs_end)
   double* uv;    // [n_obs][2] (u = col, v = row), patch pixel units
   double* xy;    // optional [n_obs][2]
   double* juv;   // optional [n_obs][juv_stride]: 2 x (6 pose | 3 point | K intr), row-major
@@ -37,31 +35,43 @@ struct ProjectArgs {
   int juv_k;     // K columns stored per row
 };
 
-// one observation: uv (and xy) to global memory, the 2 x (9 + K) record d(uv)/d(theta) to `out` (global or shared)
+// WorldToPixel + ToPixelCoordinates of observation o at the 3D point X: uv in patch pixels, xy in image pixels,
+// sc = d(uv)/d(xy) per row; with JAC the derivatives of xy (world_to_pixel)
 template <bool JAC>
-__device__ __forceinline__ void project_observation(const ProjectArgs& a, int64_t o, double* out) {
+__device__ __forceinline__ void observe(const ProjectArgs& a, int64_t o, const double X[3], double uv[2], double xy[2],
+                                        double sc[2], double Jpose[2][6], double Jpt[2][3], double Jk[2][kMaxK]) {
   const int img = a.obs_img[o];
-  const int64_t pt = a.obs_pt[o];
   const int64_t pi = a.obs_patch ? a.obs_patch[o] : o;
   const int cam = a.img_cam[img];
   const int model = a.cam_model[cam];
-  double q[4], t[3], X[3], cp[kMaxK];
+  double q[4], t[3], cp[kMaxK];
 #pragma unroll
   for (int i = 0; i < 4; ++i) q[i] = a.qvec[4 * (int64_t)img + i];
 #pragma unroll
-  for (int i = 0; i < 3; ++i) { t[i] = a.tvec[3 * (int64_t)img + i]; X[i] = a.xyz[3 * pt + i]; }
+  for (int i = 0; i < 3; ++i) t[i] = a.tvec[3 * (int64_t)img + i];
 #pragma unroll
   for (int i = 0; i < kMaxK; ++i) cp[i] = a.cam_params[(int64_t)cam * kMaxK + i];
-  double xy[2], Jpose[2][6], Jpt[2][3], Jk[2][kMaxK];
   world_to_pixel<JAC>(model, cp, q, t, X, xy, Jpose, Jpt, Jk);
   const double sx = a.scale[2 * pi], sy = a.scale[2 * pi + 1];
   const double cx = (double)a.corner[2 * pi], cy = (double)a.corner[2 * pi + 1];
-  a.uv[2 * o] = (xy[0] * sx - 0.5 - cx) * a.ups;
-  a.uv[2 * o + 1] = (xy[1] * sy - 0.5 - cy) * a.ups;
+  uv[0] = (xy[0] * sx - 0.5 - cx) * a.ups;
+  uv[1] = (xy[1] * sy - 0.5 - cy) * a.ups;
+  sc[0] = sx * a.ups; sc[1] = sy * a.ups;
+}
+
+// one observation: uv (and xy) to global memory, the 2 x (9 + K) record d(uv)/d(theta) to `out` (global or shared)
+template <bool JAC>
+__device__ __forceinline__ void project_observation(const ProjectArgs& a, int64_t o, double* out) {
+  const int64_t pt = a.obs_pt[o];
+  double X[3], uv[2], xy[2], s[2], Jpose[2][6], Jpt[2][3], Jk[2][kMaxK];
+#pragma unroll
+  for (int i = 0; i < 3; ++i) X[i] = a.xyz[3 * pt + i];
+  observe<JAC>(a, o, X, uv, xy, s, Jpose, Jpt, Jk);
+  a.uv[2 * o] = uv[0];
+  a.uv[2 * o + 1] = uv[1];
   if (a.xy) { a.xy[2 * o] = xy[0]; a.xy[2 * o + 1] = xy[1]; }
   if (JAC && out) {
     const int W = 9 + a.juv_k;
-    const double s[2] = {sx * a.ups, sy * a.ups};
 #pragma unroll
     for (int r = 0; r < 2; ++r) {
 #pragma unroll
@@ -76,8 +86,7 @@ __device__ __forceinline__ void project_observation(const ProjectArgs& a, int64_
 template <bool JAC>
 __global__ void __launch_bounds__(128) ba_project_kernel(ProjectArgs a) {
   const int64_t k = a.obs_begin + (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const int64_t end = a.n_dev ? a.obs_begin + (int64_t)*a.n_dev : a.obs_end;
-  if (k >= end) return;
+  if (k >= a.obs_end) return;
   const int64_t o = a.item_index ? a.item_index[k] : k;
   project_observation<JAC>(a, o, (JAC && a.juv) ? a.juv + o * (int64_t)a.juv_stride : nullptr);
 }
@@ -123,8 +132,6 @@ struct FmEvalArgs {
   unsigned long long* viol_count = nullptr;  // [1]
   int64_t* viol_list = nullptr;              // [viol_capacity]
   long long viol_capacity = 0;               // entries beyond it are dropped (they are reported again by the repeated pass)
-  const unsigned long long* end_dev = nullptr;   // optional: item count on the device (end = begin + *end_dev; `end` is then the
-                                                 // upper bound the grid was sized for)
   LossParams loss;
   int l2_normalize;
 };
@@ -154,6 +161,39 @@ template <typename T, int C> struct FmCfg {
   static constexpr int kWarps = kSlot <= 4096 ? PXR_FM_WARPS : (kSlot <= 8192 ? 8 : (kSlot <= 16384 ? 4 : 2));
   static constexpr int kSmem = kWarps * kFmStages * kSlot + kWarps * kFmStages * 8 + kWarps * 32 * (int)sizeof(FmAux);
 };
+
+// One TMA bulk copy of the 4x4 tap window of item x into a ring slot (completes on `bar`), whole warp.  In-range
+// columns are 4 contiguous rows of 4 taps; a window clamped at a side border falls back to 16 per-tap copies.
+template <int TAP_BYTES>
+__device__ __forceinline__ void issue_window(const FmAux& x, uint8_t* dst, uint64_t* bar, int ph, int pw, int lane) {
+  const int jc = x.col, jr = x.row;
+  if (lane == 0) mbar_expect_tx(bar, 16 * TAP_BYTES);
+  __syncwarp();
+  const bool contiguous = (jc - 1 >= 0) && (jc + 2 <= pw - 1);
+  if (contiguous) {
+    if (lane < 4) {
+      const int rr = min(max(jr - 1 + lane, 0), ph - 1);
+      bulk_g2s(dst + lane * 4 * TAP_BYTES, x.src + ((int64_t)rr * pw + (jc - 1)) * TAP_BYTES, 4 * TAP_BYTES, bar);
+    }
+  } else if (lane < 16) {
+    const int rr = min(max(jr - 1 + (lane >> 2), 0), ph - 1);
+    const int cc = min(max(jc - 1 + (lane & 3), 0), pw - 1);
+    bulk_g2s(dst + lane * TAP_BYTES, x.src + ((int64_t)rr * pw + cc) * TAP_BYTES, TAP_BYTES, bar);
+  }
+}
+
+// per-item window geometry of the projection (u, v) into a patch at src
+__device__ __forceinline__ FmAux window_geometry(double u, double v, const uint8_t* src, int64_t item, int ph, int pw) {
+  const double fu = floor(u), fv = floor(v);
+  // guard the int conversion (NaN/huge projections clamp to the border like any far-away tap)
+  FmAux x;
+  x.item = item;
+  x.col = (int)fmin(fmax(fu, -4.0), (double)pw + 4.0);
+  x.row = (int)fmin(fmax(fv, -4.0), (double)ph + 4.0);
+  x.xc = u - fu; x.xr = v - fv;
+  x.src = src;
+  return x;
+}
 
 template <typename T> struct HorizT { typedef float type; };
 template <> struct HorizT<double> { typedef double type; };
@@ -382,7 +422,7 @@ __global__ void __launch_bounds__(FmCfg<T, C>::kWarps * 32, 1) fm_eval_kernel(Fm
   }
   __syncwarp();
   const bool active = lane < ACTIVE;
-  const int64_t item_end = a.end_dev ? a.begin + (int64_t)*a.end_dev : a.end;
+  const int64_t item_end = a.end;
   const int64_t n_items = item_end - a.begin;
   const int64_t n_batches = (n_items + 31) / 32;
   const int64_t warp_global = (int64_t)blockIdx.x * kFmWarps + warp;
@@ -406,14 +446,7 @@ __global__ void __launch_bounds__(FmCfg<T, C>::kWarps * 32, 1) fm_eval_kernel(Fm
         pidx = a.item_patch ? a.item_patch[o] : o;
         ridx = a.item_ref ? a.item_ref[o] : o;
       }
-      const double fu = floor(u), fv = floor(v);
-      // guard the int conversion (NaN/huge projections clamp to the border like any far-away tap)
-      FmAux x;
-      x.item = o;
-      x.col = (int)fmin(fmax(fu, -4.0), (double)a.pw + 4.0);
-      x.row = (int)fmin(fmax(fv, -4.0), (double)a.ph + 4.0);
-      x.xc = u - fu; x.xr = v - fv;
-      x.src = a.patches + pidx * patch_bytes;
+      const FmAux x = window_geometry(u, v, a.patches + pidx * patch_bytes, o, a.ph, a.pw);
       aux[lane] = x;
       ref_idx = ridx;
       if (a.res_rect && lane < nvalid && !window_resident(a.res_rect[pidx], x.row, x.col, a.ph, a.pw)) {
@@ -424,22 +457,7 @@ __global__ void __launch_bounds__(FmCfg<T, C>::kWarps * 32, 1) fm_eval_kernel(Fm
     __syncwarp();
 
     auto issue = [&](int j, int slot) {
-      const int jc = aux[j].col, jr = aux[j].row;
-      const uint8_t* src = aux[j].src;
-      uint8_t* dst = wbase + (size_t)slot * SLOT_BYTES;
-      if (lane == 0) mbar_expect_tx(&bars[slot], SLOT_BYTES);
-      __syncwarp();
-      const bool contiguous = (jc - 1 >= 0) && (jc + 2 <= a.pw - 1);
-      if (contiguous) {
-        if (lane < 4) {
-          const int rr = min(max(jr - 1 + lane, 0), a.ph - 1);
-          bulk_g2s(dst + lane * 4 * TAP_BYTES, src + ((int64_t)rr * a.pw + (jc - 1)) * TAP_BYTES, 4 * TAP_BYTES, &bars[slot]);
-        }
-      } else if (lane < 16) {
-        const int rr = min(max(jr - 1 + (lane >> 2), 0), a.ph - 1);
-        const int cc = min(max(jc - 1 + (lane & 3), 0), a.pw - 1);
-        bulk_g2s(dst + lane * TAP_BYTES, src + ((int64_t)rr * a.pw + cc) * TAP_BYTES, TAP_BYTES, &bars[slot]);
-      }
+      issue_window<TAP_BYTES>(aux[j], wbase + (size_t)slot * SLOT_BYTES, &bars[slot], a.ph, a.pw, lane);
     };
 
     // ---- phase 2: software pipeline over the batch

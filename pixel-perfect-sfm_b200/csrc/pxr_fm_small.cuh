@@ -20,13 +20,10 @@ template <> __device__ __forceinline__ double small_tap<__half>(const __half* p)
 template <> __device__ __forceinline__ double small_tap<float>(const float* p) { return (double)*p; }
 template <> __device__ __forceinline__ double small_tap<double>(const double* p) { return *p; }
 
-template <typename T, int C, int MODE>
-static __global__ void __launch_bounds__(128) fm_eval_small_kernel(FmEvalArgs a) {
-  constexpr bool DERIV = MODE == 1;
-  const int64_t k = a.begin + (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (k >= (a.end_dev ? a.begin + (int64_t)*a.end_dev : a.end)) return;
-  const int64_t o = a.item_index ? a.item_index[k] : k;
-  const double u = a.uv[2 * o], v = a.uv[2 * o + 1];
+// one observation at the projection (u, v): red = (s, b_u, b_v, a_uu, a_uv, a_vv) (DERIV) or s; the optional
+// residual / descriptor / gradient outputs of FmEvalArgs are written here
+template <typename T, int C, bool DERIV>
+__device__ __forceinline__ void fm_small_item(const FmEvalArgs& a, int64_t o, double u, double v, double red[6]) {
   const int64_t pidx = a.item_patch ? a.item_patch[o] : o;
   const double fu = floor(u), fv = floor(v);
   const int col = (int)fmin(fmax(fu, -4.0), (double)a.pw + 4.0);
@@ -84,10 +81,22 @@ static __global__ void __launch_bounds__(128) fm_eval_small_kernel(FmEvalArgs a)
     s += r * r;
     if (DERIV) { bu += fc[ch] * r; bv += fr[ch] * r; auu += fc[ch] * fc[ch]; auv += fc[ch] * fr[ch]; avv += fr[ch] * fr[ch]; }
   }
+  red[0] = s;
+  if (DERIV) { red[1] = bu; red[2] = bv; red[3] = auu; red[4] = auv; red[5] = avv; }
+}
+
+template <typename T, int C, int MODE>
+static __global__ void __launch_bounds__(128) fm_eval_small_kernel(FmEvalArgs a) {
+  constexpr bool DERIV = MODE == 1;
+  const int64_t k = a.begin + (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= a.end) return;
+  const int64_t o = a.item_index ? a.item_index[k] : k;
+  double red[6];
+  fm_small_item<T, C, DERIV>(a, o, a.uv[2 * o], a.uv[2 * o + 1], red);
   if (a.out) {
     double* op = a.out + o * 8;
-    op[0] = s;
-    if (DERIV) { op[1] = bu; op[2] = bv; op[3] = auu; op[4] = auv; op[5] = avv; }
+    op[0] = red[0];
+    if (DERIV) { op[1] = red[1]; op[2] = red[2]; op[3] = red[3]; op[4] = red[4]; op[5] = red[5]; }
   }
 }
 
